@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py -- the hot-path benchmark of b200slam (contract: task brief, section 4).
+"""bench.py -- the hot-path benchmark of b200slam.
 
 Metric (BASELINE.json): scan matches/sec (1081-beam, +-2 m / +-20 deg) on the loop-closure
 batch workload (configs[1]: 1 query x 1000 candidate 1081-beam scans per GPU), plus the
@@ -9,6 +9,8 @@ under "graph_solve", and the map-publish step (occupancy grid from 5,000 scans) 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU path
                                                            # (oracle/_ref = unmodified karto_sdk)
+  python bench.py ... --dump-outputs DIR                   # also write what the timed path computed in its
+                                                           # last step as DIR/<name>.npy (see dump_outputs)
 
 One "step" = one pass of the hot path over one batch: every rank sweeps its shard of candidate
 chains (rasterise + exhaustive (x, y, theta) correlation + reduction for each (query, chain)
@@ -107,6 +109,22 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """--dump-outputs: writes each array as <directory>/<name>.npy.  Every input of the benchmark comes from fixed seeds,
+    so two builds run with the same arguments can be compared output for output.  Float64 values and integer counters
+    are written as float64 (exact), 8-bit cells as float32."""
+    out = {name: np.asarray(a, dtype=np.float32 if np.asarray(a).dtype == np.uint8 else np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_LIMIT_BYTES}")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def make_inputs(rank: int, n_cand: int, chain_len: int, n_query: int):
     from slam_toolbox_b200 import synth
     # same world + queries on every rank, candidates differ per rank (sharded candidate set)
@@ -191,9 +209,11 @@ def run_reference(args, rank, world):
     n_sample = N_CAND
     rates = []
     for i in range(args.warmup + args.steps):
-        rate, kind, sec, _, used = cpu_sweep(qr, qp, cr, cp, cs, n_sample, threads)
+        rate, kind, sec, resp, used = cpu_sweep(qr, qp, cr, cp, cs, n_sample, threads)
         if i >= args.warmup:
             rates.append((rate, sec))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"response": resp})
     value = float(np.mean([r for r, _ in rates]))
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -470,9 +490,10 @@ def cfg5_bench(rank: int, world: int, stream, flush, n_query: int, n_cand: int, 
     return dev_ms, e2e_ms, npairs, bool(ok), info["kernel"], float(win[1].mean())
 
 
-def graph_solve_case(sigma, steps: int, with_cpu: bool, peak_gbs: float):
+def graph_solve_case(sigma, steps: int, with_cpu: bool, peak_gbs: float, outputs: dict | None = None, tag: str = "graph"):
     """One cfg4 graph (10k nodes / 40k edges, dead-reckoned start) at one measurement-noise level, solved `steps` times on ONE
-    solver handle (like the mapper's: device buffers persist, Reset + re-adding the graph makes every solve a cold graph)."""
+    solver handle (like the mapper's: device buffers persist, Reset + re-adding the graph makes every solve a cold graph).
+    `outputs` receives the node ids and corrected poses of the last timed solve as <tag>_ids / <tag>_poses."""
     from slam_toolbox_b200 import synth, api
     g = synth.make_pose_graph(0, GRAPH_NODES, GRAPH_EDGES, sigma_xy=sigma[0], sigma_th=sigma[1])
     E = int(len(g["edge_a"]))
@@ -491,7 +512,9 @@ def graph_solve_case(sigma, steps: int, with_cpu: bool, peak_gbs: float):
         summ = s.summary
         if i > 0:
             rows.append((summ.solve_ms, wall, summ.setup_ms))
-        poses = s.GetCorrections()[1]
+        ids, poses = s.GetCorrections()
+    if outputs is not None:
+        outputs[f"{tag}_ids"], outputs[f"{tag}_poses"] = ids, poses
     ms = float(np.mean([r[0] for r in rows]))
     # what the mapper does after the NEXT loop closure (Mapper.cpp:2012-2030): one more constraint on the solved graph
     k = E - 1
@@ -538,15 +561,16 @@ def graph_solve_case(sigma, steps: int, with_cpu: bool, peak_gbs: float):
     return out
 
 
-def graph_solve_bench(steps: int, with_cpu: bool, peak_gbs: float = 6650.0):
+def graph_solve_bench(steps: int, with_cpu: bool, peak_gbs: float = 6650.0, outputs: dict | None = None):
     """cfg4 at the contract's noise level (SURVEY.md 8d: 0.05 m / 0.02 rad) and at the lower one round 1 reported."""
-    out = graph_solve_case((0.05, 0.02), steps, with_cpu, peak_gbs)
-    out["low_noise_variant"] = graph_solve_case(GRAPH_SIGMA, steps, with_cpu, peak_gbs)
+    out = graph_solve_case((0.05, 0.02), steps, with_cpu, peak_gbs, outputs, "graph")
+    out["low_noise_variant"] = graph_solve_case(GRAPH_SIGMA, steps, with_cpu, peak_gbs, outputs, "graph_low_noise")
     return out
 
 
-def occupancy_bench(steps: int, with_cpu: bool):
-    """Map publish (SURVEY.md 8f row 4): OccupancyGrid::CreateFromScans over a cfg3-sized run of 5,000 scans at 0.05 m."""
+def occupancy_bench(steps: int, with_cpu: bool, outputs: dict | None = None):
+    """Map publish (SURVEY.md 8f row 4): OccupancyGrid::CreateFromScans over a cfg3-sized run of 5,000 scans at 0.05 m.
+    `outputs` receives the grid of the last timed build: occupancy_cells, occupancy_passes, occupancy_hits."""
     from slam_toolbox_b200 import synth, api
     n_scans, res = 5000, 0.05
     run = synth.make_mapping_run(3, n_scans, world=synth.make_world(3, size=60.0), odd_readings=False)
@@ -559,6 +583,8 @@ def occupancy_bench(steps: int, with_cpu: bool):
         g.Build()
         ms.append(g.kernel_ms())
     cells, ps, ht = g.GetData(counters=True)
+    if outputs is not None:
+        outputs.update(occupancy_cells=cells, occupancy_passes=ps, occupancy_hits=ht)
     updates = int(ps.sum())
     launches = g.launch_count()
     g.close()
@@ -610,6 +636,9 @@ def main():
     ap.add_argument("--sweep-kernel", type=int, default=0, help="0 auto, 1 single-CTA kernel, 2 tiled cluster kernel (headline workload)")
     ap.add_argument("--chain-len", type=int, default=CHAIN_LEN)
     ap.add_argument("--candidates", type=int, default=N_CAND)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step as DIR/<name>.npy: "
+                    "the headline sweep's response, mean and covariance per pair (rank 0's shard), and the pose-graph poses and "
+                    "occupancy grid when those parts run")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -840,10 +869,13 @@ def main():
             line["replay"] = replay_bench(args.replay_scans, args.replay_ref_scans)
         except Exception as ex:   # the replay needs the prebuilt integration libraries
             line["replay"] = {"unavailable": str(ex)[-300:]}
+    outputs = {"response": resp_dev, "mean": mean_dev, "covariance": cov_dev}
     if not args.no_graph:
-        line["graph_solve"] = graph_solve_bench(3, not args.no_cpu, peak)
+        line["graph_solve"] = graph_solve_bench(3, not args.no_cpu, peak, outputs)
     if not args.no_map:
-        line["occupancy_grid"] = occupancy_bench(5, not args.no_cpu)
+        line["occupancy_grid"] = occupancy_bench(5, not args.no_cpu, outputs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

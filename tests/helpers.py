@@ -1,5 +1,6 @@
 """Shared fixtures for the parity tests: the parameter sets of BASELINE.json's configs and
-constructors for the three implementations (reference .so, C port oracle, CUDA product)."""
+constructors for the three implementations (reference .so, C port oracle, CUDA product), and the codec of the laser
+ranges stored in the golden fixtures."""
 from __future__ import annotations
 
 import math
@@ -74,6 +75,43 @@ def gpu_block(ranges, poses, range_threshold=None):
                                  minimum_range=LASER["min_range"], maximum_range=LASER["max_range"],
                                  range_threshold=LASER["range_threshold"] if range_threshold is None else range_threshold)
     return api.ScanBlock(ranges, poses, laser)
+
+
+def digest(a) -> str:
+    """SHA-256 of an array's bytes, NaNs canonicalised first: equal digests mean np.array_equal(..., equal_nan=True)."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a)
+    return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+# laser ranges in the golden fixtures: uint16 millimetres, three codes reserved for +inf, NaN and readings that are not a
+# whole number of millimetres (their exact float64 values are stored separately, in order)
+RANGE_INF, RANGE_NAN, RANGE_EXACT = 65535, 65534, 65533
+
+
+def pack_ranges(r):
+    r = np.asarray(r, dtype=np.float64)
+    finite = np.isfinite(r)
+    assert not (np.isinf(r) & (r < 0)).any() and (r[finite] >= 0).all() and (r[finite] < RANGE_EXACT / 1000.0).all()
+    mm = np.round(np.where(finite, r, 0.0) * 1000.0)
+    exact = finite & (mm / 1000.0 != r)
+    codes = np.where(np.isnan(r), RANGE_NAN, np.where(np.isinf(r), RANGE_INF, np.where(exact, RANGE_EXACT, mm)))
+    return codes.astype(np.uint16), r[exact]
+
+
+def unpack_ranges(codes, exact):
+    r = codes.astype(np.float64) / 1000.0
+    r[codes == RANGE_INF] = np.inf
+    r[codes == RANGE_NAN] = np.nan
+    r[codes == RANGE_EXACT] = exact
+    return r
+
+
+def golden_ranges(z, key):
+    """The ranges stored under `key` by pack_ranges (keys <key>_mm and <key>_exact)."""
+    return unpack_ranges(z[f"{key}_mm"], z[f"{key}_exact"])
 
 
 def assert_occupancy_equals_golden(g, z, name):

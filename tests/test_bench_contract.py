@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
              "dtype", "data", "config", "e2e", "gpu_launches", "cpu_baseline"}
@@ -33,3 +36,39 @@ def test_committed_round_profile_has_the_contract_keys():
     assert {"value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step"} <= set(d["e2e"])
     assert d["gpu_launches"] > 0 and d["e2e"]["h2d_bytes_per_step"] > 0 and d["e2e"]["value"] < d["value"]
     assert d["dtype"] == "u8" and d["data"] == "synthetic" and d["scaling"] == "weak"
+
+
+def test_dump_outputs_writes_float_arrays_within_the_limit(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    arrays = {"response": np.linspace(0.0, 1.0, 7), "cells": np.array([[0, 100, 255]], dtype=np.uint8),
+              "passes": np.array([3, 2 ** 31 + 1], dtype=np.uint32), "ids": np.arange(4, dtype=np.int32)}
+    bench.dump_outputs(str(tmp_path / "out"), arrays)
+    assert sorted(os.listdir(tmp_path / "out")) == ["cells.npy", "ids.npy", "passes.npy", "response.npy"]
+    for name, a in arrays.items():
+        b = np.load(tmp_path / "out" / f"{name}.npy")
+        assert b.dtype == (np.float32 if a.dtype == np.uint8 else np.float64) and np.array_equal(a, b)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 8 + 1)})
+    assert not (tmp_path / "big").exists()
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_repeat_exactly_between_runs(tmp_path):
+    """Two runs with the same arguments: the same inputs, so the same outputs, bit for bit (the sweep is exact)."""
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--candidates", "64",
+                            "--no-graph", "--no-map", "--no-cpu", "--no-rows", "--no-seq", "--no-replay", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 2 and line["gpu_launches"] > 0
+        assert sorted(os.listdir(d)) == ["covariance.npy", "mean.npy", "response.npy"]
+        dumps.append({n: np.load(d / f"{n}.npy") for n in ("response", "mean", "covariance")})
+    a, b = dumps
+    assert a["response"].shape == (64,) and a["mean"].shape == (64, 3) and a["covariance"].shape == (64, 3, 3)
+    assert all(v.dtype == np.float64 for v in a.values()) and a["response"].max() > 0
+    for n in a:
+        assert np.array_equal(a[n], b[n]), n

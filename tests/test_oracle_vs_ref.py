@@ -1,6 +1,5 @@
-"""Pins the plain-C oracle (oracle/karto_port.c) against the reference itself: the unmodified
-karto_sdk compiled into oracle/_ref/libkarto_ref.so (present in the build container; travels to the
-GPU box as a prebuilt .so) and against the committed golden fixtures generated from it."""
+"""Pins the plain-C oracle (oracle/karto_port.c) against the reference: the unmodified karto_sdk, through the committed
+golden fixtures generated from it (tests/golden/make_golden.py, tests/golden/make_reference_golden.py)."""
 import hashlib
 import math
 import os
@@ -10,15 +9,20 @@ import pytest
 
 import helpers as H
 from oracle import karto_port as P
-from oracle import karto_ref as R
 from slam_toolbox_b200 import synth
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "matcher_golden.npz")
-needs_ref = pytest.mark.skipif(not R.available(), reason="oracle/_ref/libkarto_ref.so not built")
+REF_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference_matcher_golden.npz")
 
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def golden_case(z, key):
+    """inputs of one case of reference_matcher_golden.npz"""
+    return dict(base_ranges=H.golden_ranges(z, f"{key}/base_ranges"), base_poses=z[f"{key}/base_poses"],
+                query_ranges=H.golden_ranges(z, f"{key}/query_ranges"), query_pose=z[f"{key}/query_pose"])
 
 
 def golden_cases():
@@ -56,65 +60,61 @@ def test_port_matches_golden(name):
     assert int(vol.argmax()) == z[f"{name}/volume_argmax"][0] and int(vol.max()) == z[f"{name}/volume_argmax"][1]
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [0, 1, 2])
 @pytest.mark.parametrize("cfg", ["seq", "seq_yaml", "loop"])
 def test_port_vs_reference_match(seed, cfg):
+    z, key = np.load(REF_GOLDEN), f"match/{cfg}/{seed}"
     mapper, grid = {"seq": (H.MAPPER_SEQ, H.GRID_SEQ), "seq_yaml": (H.MAPPER_SEQ, H.GRID_SEQ_YAML),
                     "loop": (H.MAPPER_LOOP, H.GRID_LOOP)}[cfg]
-    case = synth.make_sequential_case(100 + seed, buffer_len=4, inf_frac=0.03 * (seed % 2), nan_frac=0.01 * (seed == 2))
-    rm, pm = H.ref_matcher(mapper, grid), H.port_matcher(mapper, grid)
-    rb, pb = H.ref_scans(case["base_ranges"], case["base_poses"]), H.port_scans(case["base_ranges"], case["base_poses"])
-    rq, pq = H.ref_scans(case["query_ranges"], case["query_pose"], 99)[0], H.port_scans(case["query_ranges"], case["query_pose"])[0]
-    assert np.array_equal(rq.points(), pq.points, equal_nan=True)
-    for pen, refine in ((True, True), (False, False), (False, True)):
-        a, b = rm.match(rq, rb, pen, refine), pm.match(pq, pb, pen, refine)
-        assert a[0] == b[0] and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
-    g1, g2 = rm.grid(), pm.grid()
-    assert np.array_equal(g1["data"], g2["data"]) and g1["offset"] == g2["offset"]
-    assert (g1["width"], g1["stride"], g1["roi"], g1["kernel_size"]) == (g2["width"], g2["stride"], g2["roi"], g2["kernel_size"])
-    assert np.array_equal(rm.kernel(), pm.kernel())
-    o1 = rm.offsets(rq, case["query_pose"][2] + 0.01, mapper["coarse_search_angle_offset"], mapper["coarse_angle_resolution"])
-    o2 = pm.offsets(pq, case["query_pose"][2] + 0.01, mapper["coarse_search_angle_offset"], mapper["coarse_angle_resolution"])
-    assert np.array_equal(o1, o2)
+    case = golden_case(z, f"case{seed}")
+    pm = H.port_matcher(mapper, grid)
+    pb, pq = H.port_scans(case["base_ranges"], case["base_poses"]), H.port_scans(case["query_ranges"], case["query_pose"])[0]
+    assert H.digest(pq.points) == z[f"case{seed}/query_points_sha"][0]
+    for i, (pen, refine) in enumerate(((True, True), (False, False), (False, True))):
+        b = pm.match(pq, pb, pen, refine)
+        assert z[f"{key}/response"][i] == b[0] and np.array_equal(z[f"{key}/mean"][i], b[1]) and np.array_equal(z[f"{key}/cov"][i], b[2])
+    g = pm.grid()
+    assert H.digest(g["data"]) == z[f"{key}/grid_sha"][0] and g["offset"] == tuple(z[f"{key}/grid_offset"])
+    assert [g["width"], g["stride"], *g["roi"], g["kernel_size"]] == list(z[f"{key}/grid_geometry"])
+    assert np.array_equal(z[f"{key}/kernel"], pm.kernel())
+    o = pm.offsets(pq, case["query_pose"][2] + 0.01, mapper["coarse_search_angle_offset"], mapper["coarse_angle_resolution"])
+    assert H.digest(o) == z[f"{key}/offsets_sha"][0]
     vp = case["query_pose"][:2] + 0.3
-    for r_s, p_s in zip(rb, pb):
-        assert np.array_equal(rm.find_valid_points(r_s, vp), P.find_valid_points(p_s, vp), equal_nan=True)
+    assert [H.digest(P.find_valid_points(p_s, vp)) for p_s in pb] == list(z[f"{key}/valid_points_sha"])
 
 
-@needs_ref
 def test_port_vs_reference_edge_cases():
-    mapper, grid = H.MAPPER_LOOP, H.GRID_SMALL
-    rm, pm = H.ref_matcher(mapper, grid), H.port_matcher(mapper, grid)
-    case = synth.make_sequential_case(7, buffer_len=2)
-    rq, pq = H.ref_scans(case["query_ranges"], case["query_pose"], 5)[0], H.port_scans(case["query_ranges"], case["query_pose"])[0]
+    z = np.load(REF_GOLDEN)
+    pm = H.port_matcher(H.MAPPER_LOOP, H.GRID_SMALL)
+    case = golden_case(z, "edge")
+    pq = H.port_scans(case["query_ranges"], case["query_pose"])[0]
+    pb = H.port_scans(case["base_ranges"], case["base_poses"])
+
+    def same(name, b):
+        a = [z[f"edge/{name}/response"][0], z[f"edge/{name}/mean"], z[f"edge/{name}/cov"]]
+        return a[0] == b[0] and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
     # no base scans at all: zero response everywhere, every pose ties, response expansion kicks in
-    a, b = rm.match(rq, [], True, True), pm.match(pq, [], True, True)
-    assert a[0] == b[0] == 0.0 and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
+    b = pm.match(pq, [], True, True)
+    assert z["edge/empty/response"][0] == b[0] == 0.0 and same("empty", b)
     # all-invalid query readings
     bad = np.full_like(case["query_ranges"], np.inf)
-    rq2, pq2 = H.ref_scans(bad, case["query_pose"], 6)[0], H.port_scans(bad, case["query_pose"])[0]
-    rb, pb = H.ref_scans(case["base_ranges"], case["base_poses"]), H.port_scans(case["base_ranges"], case["base_poses"])
-    a, b = rm.match(rq2, rb, False, False), pm.match(pq2, pb, False, False)
-    assert a[0] == b[0] and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
+    assert same("bad_query", pm.match(H.port_scans(bad, case["query_pose"])[0], pb, False, False))
     # query far away from the base scans (nothing overlaps)
     far = case["query_pose"] + np.array([500.0, -300.0, 1.0])
-    rq3, pq3 = H.ref_scans(case["query_ranges"], far, 7)[0], H.port_scans(case["query_ranges"], far)[0]
-    a, b = rm.match(rq3, rb, True, False), pm.match(pq3, pb, True, False)
-    assert a[0] == b[0] and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
+    assert same("far_query", pm.match(H.port_scans(case["query_ranges"], far)[0], pb, True, False))
 
 
-@needs_ref
 def test_raster_order_dependence_is_reproduced():
     """SURVEY.md 7 hard part 2: with smear 0.1 @ 0.01 m the grid depends on base-scan order."""
-    case = synth.make_sequential_case(3, buffer_len=4)
-    rm, pm = H.ref_matcher(H.MAPPER_SEQ, H.GRID_SEQ_YAML), H.port_matcher(H.MAPPER_SEQ, H.GRID_SEQ_YAML)
-    rq, pq = H.ref_scans(case["query_ranges"], case["query_pose"], 9)[0], H.port_scans(case["query_ranges"], case["query_pose"])[0]
-    rb, pb = H.ref_scans(case["base_ranges"], case["base_poses"]), H.port_scans(case["base_ranges"], case["base_poses"])
+    z = np.load(REF_GOLDEN)
+    case = golden_case(z, "raster")
+    pm = H.port_matcher(H.MAPPER_SEQ, H.GRID_SEQ_YAML)
+    pq = H.port_scans(case["query_ranges"], case["query_pose"])[0]
+    pb = H.port_scans(case["base_ranges"], case["base_poses"])
     grids = []
-    for order in (slice(None), slice(None, None, -1)):
-        rm.raster(rq, rb[order]); pm.raster(pq, pb[order])
-        assert np.array_equal(rm.grid()["data"], pm.grid()["data"])
+    for order, ref_sha in zip((slice(None), slice(None, None, -1)), z["raster/grid_sha"]):
+        pm.raster(pq, pb[order])
+        assert H.digest(pm.grid()["data"]) == ref_sha
         grids.append(pm.grid()["data"])
     assert not np.array_equal(grids[0], grids[1])
 

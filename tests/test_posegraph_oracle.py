@@ -1,15 +1,17 @@
-"""Checks of the restated pose-graph oracle (oracle/posegraph.py; PARITY UNPINNED -- Ceres is not in
-the container): its building blocks against the reference's own karto code where that exists
-(LinkInfo, Matrix3::Inverse) and its minimiser against scipy.optimize.least_squares."""
+"""Checks of the restated pose-graph oracle (oracle/posegraph.py; PARITY UNPINNED -- the reference's solver is
+Ceres, which the tests do not link): its building blocks against the reference's own karto code where that exists
+(LinkInfo, Matrix3::Inverse, through tests/golden/reference_posegraph_golden.npz) and its minimiser against
+scipy.optimize.least_squares."""
+import os
+
 import numpy as np
 import pytest
 from scipy.optimize import least_squares
 
-from oracle import karto_ref as R
 from oracle import posegraph as PG
 from slam_toolbox_b200 import synth
 
-needs_ref = pytest.mark.skipif(not R.available(), reason="oracle/_ref/libkarto_ref.so not built")
+REF_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference_posegraph_golden.npz")
 
 
 def test_normalize_angle_range():
@@ -20,19 +22,15 @@ def test_normalize_angle_range():
     assert PG.normalize_angle(np.array([np.pi]))[0] == -np.pi
 
 
-@needs_ref
 def test_link_info_and_inverse_match_karto():
-    rng = np.random.default_rng(0)
-    for _ in range(20):
-        p1, p2 = rng.uniform(-5, 5, 3), rng.uniform(-5, 5, 3)
-        A = rng.normal(size=(3, 3))
-        cov = A @ A.T + 0.1 * np.eye(3)
-        d_ref, c_ref = R.link_info(p1, p2, cov)
+    z = np.load(REF_GOLDEN)
+    assert len(z["p1"]) == 20
+    for p1, p2, cov, d_ref, c_ref, inv_ref in zip(z["p1"], z["p2"], z["cov"], z["link_delta"], z["link_cov"], z["inverse"]):
         d, c = PG.link_info(p1, p2, cov)
         assert np.allclose(d[:2], d_ref[:2], atol=1e-12)
         assert abs(np.sin(d[2] - d_ref[2])) < 1e-12 and np.cos(d[2] - d_ref[2]) > 0
         assert np.allclose(c, c_ref, atol=1e-12)
-        assert np.allclose(PG.matrix3_inverse(cov), R.matrix3_inverse(cov), rtol=1e-13, atol=0)
+        assert np.allclose(PG.matrix3_inverse(cov), inv_ref, rtol=1e-13, atol=0)
 
 
 def test_sqrt_information_is_upper_cholesky_of_the_information():
