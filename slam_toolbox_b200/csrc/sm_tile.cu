@@ -12,11 +12,13 @@
 //   * the pose volume is cut into V angle CHUNKS; a thread-block CLUSTER of C CTAs shares one pair and CTA r
 //     owns chunks r, r + C, ... (perfectly balanced: every angle has the same beams);
 //   * the parity sub-grid is cut into row BANDS (band rows + a halo of one pose-window height), one band is
-//     resident at a time, beams are grouped by (angle, parity phase, band, alignment);
+//     resident at a time, FAST beams form one stream per (angle, parity phase, band);
 //   * the beam-descriptor block of every (chunk, phase, band) STAGE is streamed into shared memory by
 //     cp.async.bulk (TMA, 1-D) completing on an mbarrier, double buffered: the block of stage s + 1 lands
-//     while stage s is being correlated; the hot loop reads descriptors with broadcast LDS.64;
-//   * warp items (angle, x-tile, y-tile, alignment) come from a dynamic shared-memory queue;
+//     while stage s is being correlated; the hot loop reads descriptors with broadcast LDS.128;
+//   * the FAST beam loop runs on the integer tensor cores (mma.sync m16n8k32 u8): the word loads are the A fragments, the beams'
+//     weights and byte alignments form B;
+//   * warp items (FAST: angle, slot group, word range; EDGE: angle, alignment, y-tile, x-tile) come from a dynamic shared-memory queue;
 //   * the reduction (CorrelateScan M.cpp:775-829, ComputePositionalCovariance M.cpp:893-933) is distributed:
 //     every CTA reduces its chunks to (best, tie list, per-cell max image), the images and tie lists are
 //     combined through DISTRIBUTED SHARED MEMORY by a leader CTA that rotates from pair to pair, and a split
@@ -42,7 +44,8 @@ namespace b200 {
 
 constexpr int kRowTiles = 6;           // row tiles of 8 rows per thread: one y-tile = 48 poses
 constexpr int kYTile = 8 * kRowTiles;
-constexpr int kChunkBeams = 640;       // beams accumulated in 16-bit fields before a flush (640 * 100 < 65536)
+constexpr int kChunkBeams = 640;       // EDGE beams accumulated in 16-bit fields before a flush (640 * 100 < 65536)
+constexpr int kTileSlots = 6;          // FAST items: sub-grid words W (MMA slot groups of 16 poses) per warp item
 
 // ------------------------------------------------------------------------------------------
 // PTX helpers: mbarrier, bulk async copy (TMA 1-D), cluster barrier, distributed shared memory
@@ -108,6 +111,14 @@ __device__ __forceinline__ uint32_t lds_u32(uint32_t a)
   uint32_t v;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
   return v;
+}
+
+// D += A B on the integer tensor cores: m16n8k32, A (16 x 32) and B (32 x 8) unsigned bytes, s32 accumulators
+__device__ __forceinline__ void mma_u8(int (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1)
+{
+  asm("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+      : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
+      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
 __device__ __forceinline__ uint32_t even_bytes_t(uint32_t w) { return __byte_perm(w, 0, 0x4240); }   // [b0, 0, b2, 0]
@@ -302,123 +313,88 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_sweep_tile(SweepDev d, Tile
       }
       mbar_wait(bar0 + 8 * (cnt & 1), (cnt >> 1) & 1);
       const unsigned char * stg = s_raw + f.off_stage + (size_t)(cnt & 1) * f.stage_bytes;
+      // block: [per angle (first step, end step, owns the angle's EDGE beams) | angles by descending stream length | 64-byte steps]
       const int32_t * tbl = reinterpret_cast<const int32_t *>(stg);
-      const uint8_t * order = stg + (size_t)e.na * 48;   // (angle, alignment) groups by descending length: the shared queue hands out long items first
-      const uint16_t * pay = reinterpret_cast<const uint16_t *>(stg + (((size_t)e.na * 52 + 15) & ~(size_t)15));
-      // ---- FAST + EDGE beams: warp items (angle, alignment, y-tile, x-tile) from the shared queue ----
+      const uint8_t * order = stg + (size_t)e.na * 12;
+      const uint4 * steps = reinterpret_cast<const uint4 *>(stg + (((size_t)e.na * 13 + 15) & ~(size_t)15));
+      // ---- warp items from the shared queue: FAST (angle, 16-row slot group, word range), then EDGE (angle, alignment,
+      //      y-tile, x-tile) ----
+      const int per_angle = f.ygroups * f.wranges;
+      const int fast_items = e.na * per_angle;
       const int tiles = f.ytiles * f.xtiles;
-      const int nitems = e.na * 4 * tiles;
-      const bool has_edge = (e.flags & kSeqHasEdge) != 0;
+      const int nitems = fast_items + ((e.flags & kSeqHasEdge) ? e.na * 4 * tiles : 0);
       for (;;) {
         int item = 0;
         if (lane == 0) item = atomicAdd(&sh.ctr[cnt & 1], 1);
         item = __shfl_sync(0xffffffffu, item, 0);
         if (item >= nitems) break;
-        const int gi = item / tiles, ti = item - gi * tiles;
-        const int g = order[gi];
-        const int al = g >> 2, m = g & 3;
-        const int yt = ti / f.xtiles, xt = ti - yt * f.xtiles;
+        if (item < fast_items) {
+          // FAST beams on the integer tensor cores: per 8-beam step one m16n8k32 u8 MMA per slot W of the item.  A row = pose
+          // slot (rows g and g + 8 of the slot group at sub-grid word W), k = 4 * beam + byte: the lane's LDS.32 of a beam's
+          // word IS its A fragment.  B[4b + j][n] = w_b * [j - m_b + 4 == n], so C[slot][n] = sum_b w_b * cell(c_b + 4W - 4 + n)
+          // is the exact integer sum of pose x = 4W - 4 + n (n = 1..7; one stream serves every byte alignment m_b).
+          const int gi = item / per_angle, ti = item - gi * per_angle;
+          const int al = order[gi];
+          const int s0 = tbl[3 * al], s1 = tbl[3 * al + 1];
+          if (s0 == s1) continue;
+          const int yg = ti / f.wranges, wr = ti - yg * f.wranges;
+          const int g = lane >> 2, t4 = lane & 3;
+          uint32_t base = smem_u32(S8) + (uint32_t)(((16 * yg + g) * pitch_w + kTileSlots * wr) * 4);
+          asm volatile("" : "+r"(base));
+          // B fragment (k = 4 t4 + j, column n = g) of a beam whose weight sits in byte m of V: byte j takes byte j + 4 - g of V
+          uint32_t sel = 0;
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const int k = j + 4 - g;
+            sel |= (uint32_t)((k >= 0 && k <= 3) ? k : 4) << (4 * j);
+          }
+          int acc[kTileSlots][4];
+#pragma unroll
+          for (int s = 0; s < kTileSlots; ++s) acc[s][0] = acc[s][1] = acc[s][2] = acc[s][3] = 0;
+          // the lane's descriptor: byte offsets and V words of beams t4 and t4 + 4 (the 4 beams of a k-quad have distinct word
+          // offsets mod 4, the row pitch is 4 x odd words: the 32 lanes of every load hit 32 distinct banks)
+          const uint4 * de = steps + 4 * s1;
+          for (const uint4 * dp = steps + 4 * s0 + t4; dp < de; dp += 4) {
+            const uint4 dd = *dp;
+            const uint32_t oa = base + dd.x, ob = base + dd.y;
+            const uint32_t b0 = __byte_perm(dd.z, 0, sel), b1 = __byte_perm(dd.w, 0, sel);
+#pragma unroll
+            for (int s = 0; s < kTileSlots; ++s)
+              mma_u8(acc[s], lds_u32(oa + 4 * s), lds_u32(oa + 4 * s + 8 * pitchB), lds_u32(ob + 4 * s), lds_u32(ob + 4 * s + 8 * pitchB),
+                     b0, b1);
+          }
+          // once per item: C (rows g / g + 8, columns 2 t4 / 2 t4 + 1) into the accumulators; slots W and W + 1 share poses
+          // 4W + 1 .. 4W + 3, the shared-memory atomics add both
+          int32_t * Arow = A + (size_t)(e.a0 + al - chunk_a0) * P;
+#pragma unroll
+          for (int s = 0; s < kTileSlots; ++s) {
+            const int x = 4 * (kTileSlots * wr + s) - 4 + 2 * t4;
+#pragma unroll
+            for (int hh = 0; hh < 2; ++hh) {
+              const int y = 16 * yg + g + 8 * hh;
+              if (y >= nY) continue;
+              if (acc[s][2 * hh] && (unsigned)x < (unsigned)nX) atomicAdd(Arow + y * nX + x, acc[s][2 * hh]);
+              if (acc[s][2 * hh + 1] && (unsigned)(x + 1) < (unsigned)nX) atomicAdd(Arow + y * nX + x + 1, acc[s][2 * hh + 1]);
+            }
+          }
+          continue;
+        }
+        // EDGE beams (window partly outside the grid) of one (angle, alignment, tile): word loads with rows / words outside the
+        // band allocation masked (they index outside [0, data_size) or wrap in the reference; the wrapped part is added from the
+        // wrap2 list below).  Rows / words inside the allocation but beyond the valid cells are zero padding.
+        const int ei = item - fast_items;
+        const int gi = ei / tiles, ti = ei - gi * tiles;
+        const int al = gi >> 2, m = gi & 3;
+        if (!tbl[3 * al + 2]) continue;   // the angle's stream started in an earlier block, which took its EDGE beams
         const int a = e.a0 + al;
+        const int32_t * es = f.edge_start + (((size_t)q * nA + a) * 4 * nb + e.stage) * 4 + m;
+        int eb = es[0];
+        const int ee = es[1];
+        if (eb == ee) continue;
+        const int yt = ti / f.xtiles, xt = ti - yt * f.xtiles;
         int32_t * Arow = A + (size_t)(a - chunk_a0) * P;
         const int ybase = y_l + kYTile * yt;
-       {
-        int b = tbl[(al * 4 + m) * 3 + 0];
-        const int mb = tbl[(al * 4 + m) * 3 + 1], me = tbl[(al * 4 + m) * 3 + 2];
-        const int pe = mb;   // plain entries [b, pe) (list start 4-aligned), multi entries (offset, multiplicity) pairs [mb, me)
-        int eb = 0, ee = 0;
-        if (has_edge) {
-          const int32_t * es = f.edge_start + (((size_t)q * nA + a) * 4 * nb + e.stage) * 4 + m;
-          eb = es[0]; ee = es[1];
-        }
-        if (b == pe && mb == me && eb == ee) break;   // the groups are sorted by length: every later item is empty too
-        uint32_t base = smem_u32(S8) + (uint32_t)(((y_l + kYTile * yt) * pitch_w + 4 * xt + j_l) * 4);   // shared-window address
-        asm volatile("" : "+r"(base));   // one opaque register: every descriptor then costs PRMT + IMAD (no re-association of the sum)
-        // Idle lanes of the last y-tile (rows beyond the last pose) read past the band's nY-row halo, at most 47 rows into the
-        // accumulator region that follows S in shared memory: in bounds, and their sums are dropped at the flush (y >= nY) --
-        // so a band needs a halo of nY rows, not of whole y-tiles, and the row offsets stay warp-uniform (LDS [R + UR]).
         const int x0 = 4 * (4 * xt + j_l) - m;
-        auto flush = [&](const uint32_t (&T0)[kRowTiles], const uint32_t (&T1)[kRowTiles]) {
-          uint32_t any = 0;
-#pragma unroll
-          for (int r = 0; r < kRowTiles; ++r) any |= T0[r] | T1[r];
-          if (!__any_sync(0xffffffffu, any != 0)) return;
-#pragma unroll
-          for (int r = 0; r < kRowTiles; ++r) {
-            const int y = ybase + 8 * r;
-            if (y >= nY || (T0[r] | T1[r]) == 0) continue;
-            int32_t * dst = Arow + y * nX + x0;
-            const int v0 = T0[r] & 0xFFFF, v1 = T1[r] & 0xFFFF, v2 = T0[r] >> 16, v3 = T1[r] >> 16;
-            if (v0 && (unsigned)(x0 + 0) < (unsigned)nX) atomicAdd(dst + 0, v0);
-            if (v1 && (unsigned)(x0 + 1) < (unsigned)nX) atomicAdd(dst + 1, v1);
-            if (v2 && (unsigned)(x0 + 2) < (unsigned)nX) atomicAdd(dst + 2, v2);
-            if (v3 && (unsigned)(x0 + 3) < (unsigned)nX) atomicAdd(dst + 3, v3);
-          }
-        };
-        bool multi_done = (mb == me);
-        if (b < pe || !multi_done) {
-          do {
-            const int ce = min(pe, b + kChunkBeams);
-            uint32_t T0[kRowTiles], T1[kRowTiles];
-#pragma unroll
-            for (int r = 0; r < kRowTiles; ++r) { T0[r] = 0; T1[r] = 0; }
-            for (; b + 3 < ce; b += 4) {   // 4 beams: one broadcast LDS.64 of descriptors, two byte-wise pair sums, one 3-input add per field
-              const uint2 dd = *reinterpret_cast<const uint2 *>(pay + b);
-              // 16-bit word offsets -> byte addresses: one PRMT (half-word extract) + one shift-add each
-              const uint32_t o0 = base + 4u * __byte_perm(dd.x, 0, 0x4410), o1 = base + 4u * __byte_perm(dd.x, 0, 0x4432);
-              const uint32_t o2 = base + 4u * __byte_perm(dd.y, 0, 0x4410), o3 = base + 4u * __byte_perm(dd.y, 0, 0x4432);
-#pragma unroll
-              for (int r = 0; r < kRowTiles; ++r) {
-                const uint32_t wa = lds_u32(o0 + r * 8 * pitchB) +
-                                    lds_u32(o1 + r * 8 * pitchB);
-                const uint32_t wb = lds_u32(o2 + r * 8 * pitchB) +
-                                    lds_u32(o3 + r * 8 * pitchB);
-                T0[r] = T0[r] + even_bytes_t(wa) + even_bytes_t(wb);
-                T1[r] = T1[r] + odd_bytes_t(wa) + odd_bytes_t(wb);
-              }
-            }
-            for (; b + 1 < ce; b += 2) {
-              const uint32_t dd = *reinterpret_cast<const uint32_t *>(pay + b);
-              const uint32_t o0 = base + ((dd & 0xFFFFu) << 2), o1 = base + ((dd >> 16) << 2);
-#pragma unroll
-              for (int r = 0; r < kRowTiles; ++r) {
-                const uint32_t w = lds_u32(o0 + r * 8 * pitchB) +
-                                   lds_u32(o1 + r * 8 * pitchB);
-                T0[r] += even_bytes_t(w);
-                T1[r] += odd_bytes_t(w);
-              }
-            }
-            if (b < ce) {
-              const uint32_t o0 = base + ((uint32_t)pay[b] << 2);
-#pragma unroll
-              for (int r = 0; r < kRowTiles; ++r) {
-                const uint32_t w = lds_u32(o0 + r * 8 * pitchB);
-                T0[r] += even_bytes_t(w);
-                T1[r] += odd_bytes_t(w);
-              }
-              ++b;
-            }
-            if (b == pe && !multi_done) {
-              // beams that share one grid cell: one load, fields times k (the host only builds multi entries when the
-              // whole group's weight fits one flush)
-              for (int k = mb; k < me; k += 2) {
-                const uint32_t dm = *reinterpret_cast<const uint32_t *>(pay + k);
-                const uint32_t o0 = base + ((dm & 0xFFFFu) << 2);
-                const uint32_t kk = dm >> 16;
-#pragma unroll
-                for (int r = 0; r < kRowTiles; ++r) {
-                  const uint32_t w = lds_u32(o0 + r * 8 * pitchB);
-                  T0[r] += even_bytes_t(w) * kk;
-                  T1[r] += odd_bytes_t(w) * kk;
-                }
-              }
-              multi_done = true;
-            }
-            flush(T0, T1);
-          } while (b < pe || !multi_done);
-        }
-        // EDGE beams of this group (window partly outside the grid): the same word loads with rows / words outside the
-        // band allocation masked (they index outside [0, data_size) or wrap in the reference; the wrapped part is added
-        // from the wrap2 list below).  Rows / words inside the allocation but beyond the valid cells are zero padding.
         while (eb < ee) {
           const int ce = min(ee, eb + kChunkBeams);
           uint32_t T0[kRowTiles], T1[kRowTiles];
@@ -441,9 +417,23 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_sweep_tile(SweepDev d, Tile
             }
           }
           eb = ce;
-          flush(T0, T1);
+          // 16-bit fields into the accumulators
+          uint32_t any = 0;
+#pragma unroll
+          for (int r = 0; r < kRowTiles; ++r) any |= T0[r] | T1[r];
+          if (!__any_sync(0xffffffffu, any != 0)) continue;
+#pragma unroll
+          for (int r = 0; r < kRowTiles; ++r) {
+            const int y = ybase + 8 * r;
+            if (y >= nY || (T0[r] | T1[r]) == 0) continue;
+            int32_t * dst = Arow + y * nX + x0;
+            const int v0 = T0[r] & 0xFFFF, v1 = T1[r] & 0xFFFF, v2 = T0[r] >> 16, v3 = T1[r] >> 16;
+            if (v0 && (unsigned)(x0 + 0) < (unsigned)nX) atomicAdd(dst + 0, v0);
+            if (v1 && (unsigned)(x0 + 1) < (unsigned)nX) atomicAdd(dst + 1, v1);
+            if (v2 && (unsigned)(x0 + 2) < (unsigned)nX) atomicAdd(dst + 2, v2);
+            if (v3 && (unsigned)(x0 + 3) < (unsigned)nX) atomicAdd(dst + 3, v3);
+          }
         }
-       }
       }
       if (e.flags & kSeqNewStage) {
         // ---- wrapped part of EDGE beams (row parity flipped list): poses whose column left [0, stride) by less than a
@@ -536,7 +526,9 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_sweep_tile(SweepDev d, Tile
         // ordered tie list: poses with DoubleEqual(response, best) in array order (M.cpp:807-817); every thread owns a
         // contiguous run of cells so that ranks follow array order
         const int per = (P + kTileThreads - 1) / kTileThreads;
-        const int p0 = min(P, tid * per), p1 = min(P, p0 + per);
+        int t_own;   // the thread index read here, not the kernel-wide one: ptxas kept tid * per live across the beam loop (a spill)
+        asm volatile("mov.u32 %0, %%tid.x;" : "=r"(t_own));
+        const int p0 = min(P, t_own * per), p1 = min(P, p0 + per);
         int c = 0;
         for (int p = p0; p < p1; ++p) {
           const int x = p % nX, y = p / nX;
@@ -744,9 +736,16 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
     for (int k = 1; k < nY; ++k) if (pl.ys[k] != pl.ys[0] + 2 * k) return bail(7);
   }
   // ---- geometry of one parity sub-grid ----
-  int pitch_w = (g.stride / 2 + 16 + 3) / 4;             // sub-grid row + the 3-word overhang of the last x-tile
-  while ((pitch_w & 7) != 4) ++pitch_w;                  // 8 rows x 4 words of a warp hit 32 distinct banks
+  // Row pitch: a sub-grid row (stride / 2 bytes) + 16 bytes, rounded up to 4 x odd words so that the 8 rows x 4 words of an
+  // EDGE load, and the 8 rows x 4 word residues of a FAST k-quad load, hit 32 distinct banks (76 / 92 / 116 / 132 words at the
+  // shipped geometries).  A FAST item reads kTileSlots * wranges words from a beam's word on (an EDGE item 4 * xtiles, masked
+  // to the pitch), which can run past the row's end: those bytes only feed poses x >= nX, which the flush drops, and past
+  // the last allocated row they stay inside the allocation by the overrun below.
+  int pitch_w = (g.stride / 2 + 16 + 3) / 4;
+  while ((pitch_w & 7) != 4) ++pitch_w;
   const int xtiles = (nX + 3 + 15) / 16, ytiles = (nY + kYTile - 1) / kYTile;
+  // FAST slots: word W serves poses 4W - 3 .. 4W + 3, so words 0 .. (nX + 2) / 4 cover x = 0 .. nX - 1
+  const int ygroups = (nY + 15) / 16, wranges = ((nX + 2) / 4 + 1 + kTileSlots - 1) / kTileSlots;
   const int rows_valid = (g.height + 1) / 2;
   const int halo = nY + 2;                               // rows a beam window reaches below its base row (idle row tiles are clamped) + the wrapped row
   const int base_rows = std::max(1, rows_valid - nY + 1);   // distinct base rows of beams whose window is inside the grid
@@ -775,25 +774,29 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
     const int nAc = (nA + V - 1) / V;
     if ((nA + nAc - 1) / nAc != V || nAc > 63) continue;   // same chunk size as a smaller V; group ids are bytes
     const int a_bytes = (nAc * P * 4 + 15) & ~15;
-    // staging buffer: header + 1.5 x the average descriptor bytes of a (chunk, phase) block, at least one angle's worst case
-    const int one_angle = 52 + 2 * n + 64;
-    int stage = 16 + nAc * 52 + (nAc * n * 2 * 3) / 8 + 64 * nAc;
-    stage = std::max(stage, one_angle + 64);
-    stage = (stage + 127) & ~127;
-    const int s_avail = budget - a_bytes - probs_bytes - 2 * stage;
-    if (s_avail <= 0) continue;
-    int rows_avail = s_avail / (pitch_w * 4);
-    if ((long)rows_avail * pitch_w > 65535) rows_avail = 65535 / pitch_w;   // descriptors are 16-bit word offsets
-    int B = rows_avail - halo;
-    if (B < 8) continue;
-    B = std::min(B, base_rows);
-    const int nbv = (base_rows + B - 1) / B;
-    B = (base_rows + nbv - 1) / nbv;                     // even bands
+    // staging buffer: header + about the descriptor bytes of a (chunk, phase, band) block (8 B per entry, n / 4 beams per phase
+    // and band less the beams merged into weights, plus the residue padding); a longer block is split at a step boundary.  The
+    // size depends on the number of bands and the bands on what the buffers leave: one refinement with the first pass's bands.
+    int stage = 0, B = 0, nbv = 1;
+    bool fits = true;
+    for (int pass = 0; pass < 2 && fits; ++pass) {
+      stage = 16 + nAc * 13 + (nAc * n * 3) / (2 * nbv) + 64 * nAc;
+      stage = std::max(stage, 16 + 13 + 64 * 16);
+      stage = (stage + 127) & ~127;
+      const int s_avail = budget - a_bytes - probs_bytes - 2 * stage;
+      B = s_avail / (pitch_w * 4) - halo;
+      if (s_avail <= 0 || B < 8) { fits = false; break; }
+      B = std::min(B, base_rows);
+      nbv = (base_rows + B - 1) / B;
+      B = (base_rows + nbv - 1) / nbv;                   // even bands
+    }
+    if (!fits) continue;
     // cost of one pair on one CTA, in thread-instructions: rasters (4 phases per chunk and band) + the beam loop per angle
-    // the accumulator flush of every (angle, stage, alignment, tile) item (~100 warp instructions each, 32 warps) and the fixed
+    // the accumulator flush of every (angle, stage, slot group, word range) item (~100 warp instructions each, 32 warps) and the fixed
     // cost of a stage (clear + raster + three barriers, ~3 us) are what make extra bands expensive (measured: V 1 x 3 bands at
-    // 4 m / 12 m runs 13 % slower than V 2 x 1 band)
-    const long w_angle = (long)((double)P * n * 0.8 / kTileThreads) + 4L * nbv * (4L * xtiles * ytiles * 100 / 32);
+    // 4 m / 12 m runs 13 % slower than V 2 x 1 band).  0.4 per lookup: fitted to the tensor-core loop's kernel times at V = 2 ... 11
+    // chunks, 4 m / 12 m (profiles/r3_tile_sweep.jsonl; the byte-unpack loop it replaced took 0.8)
+    const long w_angle = (long)((double)P * n * 0.4 / kTileThreads) + 4L * nbv * ((long)ygroups * wranges * 100 / 32);
     const long w_raster = 4 * (700 + 3L * std::min(B + halo, rows_valid + halo - nY) * pitch_w / kTileThreads);
     const long cost = (long)((V + Cc - 1) / Cc) * (nbv * w_raster + nAc * w_angle);
     if (bestCost < 0 || cost < bestCost) { bestCost = cost; bestV = V; bestNb = nbv; bestB = B; bestStage = stage; }
@@ -806,7 +809,7 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
   const size_t s_bytes = ((size_t)alloc_rows * pitch_w * 4 + 15) & ~(size_t)15;
   const size_t a_bytes = ((size_t)nAc * P * 4 + 15) & ~(size_t)15;
   T.C = C; T.V = V; T.nAc = nAc; T.nbands = nbands; T.band_rows = B; T.alloc_rows = alloc_rows; T.pitch_w = pitch_w;
-  T.xtiles = xtiles; T.ytiles = ytiles; T.stage_bytes = stage_bytes;
+  T.xtiles = xtiles; T.ytiles = ytiles; T.ygroups = ygroups; T.wranges = wranges; T.stage_bytes = stage_bytes;
   T.int_ties = int_ties;
   {
     // distinct non-zero smear values, ascending; up to 4 -> levelled (atomic-free) raster
@@ -824,9 +827,11 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
   if (T.off_cells + 2 * (size_t)cell_cap * 4 + sizeof(TileShared) + 64 > 227 * 1024) cell_cap = 0;
   T.cell_cap = cell_cap;
   size_t smem = T.off_cells + 2 * (size_t)cell_cap * 4;
-  // idle lanes of the last y-tile read up to (48 ytiles - nY) rows past the band (see the kernel): keep those reads inside the
-  // allocation even when everything behind S is small (tiny search windows)
-  const size_t overrun = (size_t)(kYTile * ytiles - nY + 1) * pitch_w * 4;
+  // reads past the last allocated row: idle lanes of the last y-tile read up to (48 ytiles - nY) rows past the band (EDGE), the
+  // last slot group up to (16 ygroups - nY) rows plus the words of a word range (FAST): keep them inside the allocation even when
+  // everything behind S is small (tiny search windows)
+  const size_t overrun = std::max((size_t)(kYTile * ytiles - nY + 1) * pitch_w * 4,
+                                  ((size_t)(16 * ygroups - nY + 1) * pitch_w + (size_t)kTileSlots * wranges) * 4);
   if (smem - s_bytes < overrun) smem = s_bytes + overrun;
   if (smem + sizeof(TileShared) + 64 > 227 * 1024) return bail(5);
 
@@ -839,10 +844,12 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
   std::vector<int32_t> wrap2, wrap2_start((size_t)nq * nA * nstage + 1, 0);
   std::vector<int32_t> slow, slow_start((size_t)nq * (nA + 1), 0);
   int n_fast = 0, n_edge = 0;
-  std::vector<std::vector<uint16_t>> grp((size_t)nA * nstage * 4);
+  std::vector<std::vector<uint32_t>> grp((size_t)nA * nstage);   // FAST beams: band word offset << 2 | alignment
   std::vector<std::vector<int32_t>> egrp((size_t)nA * nstage * 4), wgrp((size_t)nA * nstage);
   blob.reserve((size_t)nq * nA * n * 2 + 4096);
-  struct Encoded { int32_t tbl[12]; std::vector<uint16_t> pay; };
+  // one FAST stream per (angle, stage): 8-beam steps of 64 bytes, lane quad t4 reads {byte offset of beam t4, of beam t4 + 4,
+  // V of beam t4, of beam t4 + 4} with V = weight << 8 * alignment
+  struct Encoded { int steps; std::vector<uint32_t> pay; };
   std::vector<Encoded> enc((size_t)nA * nstage);
   std::vector<std::vector<int32_t>> slow_a(nA);
   std::vector<int> nfast_a(nA), nedge_a(nA);
@@ -851,8 +858,8 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
     const int X0 = pl.xs[0], Y0 = pl.ys[0];
     // one host-pool task per angle: classify its beams, then sort / run-length encode its groups stage by stage
     auto one_angle = [&](int a) {
-      for (int k = 0; k < nstage * 4; ++k) { grp[(size_t)a * nstage * 4 + k].clear(); egrp[(size_t)a * nstage * 4 + k].clear(); }
-      for (int k = 0; k < nstage; ++k) wgrp[(size_t)a * nstage + k].clear();
+      for (int k = 0; k < nstage * 4; ++k) egrp[(size_t)a * nstage * 4 + k].clear();
+      for (int k = 0; k < nstage; ++k) { grp[(size_t)a * nstage + k].clear(); wgrp[(size_t)a * nstage + k].clear(); }
       slow_a[a].clear();
       int nf = 0, ne = 0;
       for (int i = 0; i < n; ++i) {
@@ -865,7 +872,7 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
           const int pp = Xb & 1, pq = Yb & 1, c = Xb >> 1, r = Yb >> 1;
           const int band = std::min(r / B, nbands - 1);
           const int wo = (r - band * B) * pitch_w + (c >> 2);
-          grp[((size_t)a * nstage + (pq * 2 + pp) * nbands + band) * 4 + (c & 3)].push_back((uint16_t)wo);
+          grp[(size_t)a * nstage + (pq * 2 + pp) * nbands + band].push_back(((uint32_t)wo << 2) | (uint32_t)(c & 3));
           ++nf;
         } else if (Xb >= -g.stride && Xb + 2 * (nX - 1) < 2 * g.stride && Xb > -32768 && Xb < 32767 && Yb > -32768 && Yb < 32767) {
           // EDGE beam: at most one row wrap.  Primary entry in the beam's own phase; if some column leaves [0, stride), a
@@ -895,41 +902,38 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
         }
       }
       nfast_a[a] = nf; nedge_a[a] = ne;
-      // the angle's groups of every stage: table of (plain begin, multi begin, multi end) per alignment, relative to the
-      // angle's own payload (whose start is 4-entry aligned in the block), and the payload
+      // the angle's stream of every stage.  Beams that land in the same cell become one entry whose weight is their count (entries
+      // of at most 255: B holds bytes).  Entries are bucketed by word offset mod 4 and a k-quad takes one entry of each residue
+      // (zero-weight entries at word `residue` of row 0 fill the shorter buckets); the stream is padded to whole 8-beam steps.
       for (int sg = 0; sg < nstage; ++sg) {
-        Encoded & E = enc[(size_t)a * nstage + sg];
-        std::vector<uint16_t> & pay = E.pay;
-        pay.clear();
-        for (int m = 0; m < 4; ++m) {
-          std::vector<uint16_t> & gk = grp[((size_t)a * nstage + sg) * 4 + m];
-          std::sort(gk.begin(), gk.end());
-          while (pay.size() & 3) pay.push_back(0);   // the plain list is read with 64-bit loads
-          const int pb = (int)pay.size();
-          // run-length encode: beams that land in the same cell share a descriptor.  Entries with multiplicity >= 3 go to the
-          // group's multi list (one load, fields multiplied), provided the whole group fits one flush.
-          const bool dedup = !h->no_dedup && gk.size() <= (size_t)kChunkBeams;
-          std::vector<std::pair<uint16_t, uint16_t>> multi;
-          for (size_t i = 0; i < gk.size();) {
-            size_t j = i;
-            while (j < gk.size() && gk[j] == gk[i]) ++j;
-            const size_t cnt = j - i;
-            if (dedup && cnt >= 3) multi.emplace_back(gk[i], (uint16_t)cnt);
-            else for (size_t t = 0; t < cnt; ++t) pay.push_back(gk[i]);
-            i = j;
+        std::vector<uint32_t> & gk = grp[(size_t)a * nstage + sg];
+        std::sort(gk.begin(), gk.end());
+        std::vector<uint32_t> bk[4][2];   // per residue: byte offsets, V words
+        for (size_t i = 0; i < gk.size();) {
+          size_t j = i;
+          while (j < gk.size() && gk[j] == gk[i]) ++j;
+          const uint32_t wo = gk[i] >> 2, m = gk[i] & 3;
+          for (size_t t = i; t < j;) {
+            const uint32_t w = h->no_dedup ? 1u : (uint32_t)std::min<size_t>(j - t, 255);
+            bk[wo & 3][0].push_back(4u * wo);
+            bk[wo & 3][1].push_back(w << (8 * m));
+            t += w;
           }
-          // the multi list (offset, multiplicity pairs, read as 32-bit words) starts where the plain list ends: keep that
-          // index even by moving an odd plain list's last entry into the multi list with multiplicity 1
-          if (((int)pay.size() - pb) & 1) {
-            const uint16_t last = pay.back();
-            pay.pop_back();
-            multi.emplace_back(last, (uint16_t)1);
-          }
-          const int mb = (int)pay.size();
-          for (auto & mk : multi) { pay.push_back(mk.first); pay.push_back(mk.second); }
-          E.tbl[3 * m + 0] = pb; E.tbl[3 * m + 1] = mb; E.tbl[3 * m + 2] = (int)pay.size();
+          i = j;
         }
-        while (pay.size() & 3) pay.push_back(0);
+        size_t quads = 0;
+        for (int r = 0; r < 4; ++r) quads = std::max(quads, bk[r][0].size());
+        quads = (quads + 1) & ~(size_t)1;
+        Encoded & E = enc[(size_t)a * nstage + sg];
+        E.steps = (int)(quads / 2);
+        E.pay.assign(quads * 8, 0u);
+        for (size_t qd = 0; qd < quads; ++qd)
+          for (int r = 0; r < 4; ++r) {
+            const bool real = qd < bk[r][0].size();
+            uint32_t * d = E.pay.data() + (qd / 2) * 16 + r * 4 + (qd & 1);
+            d[0] = real ? bk[r][0][qd] : 4u * (uint32_t)r;
+            d[2] = real ? bk[r][1][qd] : 0u;
+          }
       }
     };
     host_parallel_for(nA, one_angle);
@@ -950,61 +954,63 @@ bool build_tile_tables(b200sm * h, SweepHost & S, cudaStream_t st)
           edge.insert(edge.end(), ev.begin(), ev.end());
         }
       }
-    std::vector<uint16_t> pay;
-    std::vector<int32_t> tbl;
+    struct Seg { int a, k0, k1; };
+    std::vector<Seg> segs;
     for (int r = 0; r < C; ++r) {
       seq_start[(size_t)q * C + r] = (int32_t)seq.size();
       for (int v = r; v < V; v += C) {
         const int ca0 = v * nAc, cna = std::min(nAc, nA - ca0);
         for (int sg = 0; sg < nstage; ++sg) {
-          // sub-blocks: as many angles as fit one staging buffer
-          int a = ca0;
+          // sub-blocks: as many steps as fit one staging buffer; an angle's stream may continue in the next sub-block (the
+          // accumulators are sums, the EDGE beams go with the angle's first part)
+          int a = ca0, k = 0;
           bool first_sub = true;
           do {
-            tbl.clear(); pay.clear();
-            int na = 0;
-            while (a + na < ca0 + cna) {
-              const Encoded & E = enc[(size_t)(a + na) * nstage + sg];
-              const size_t hdr = (((size_t)(na + 1) * 52) + 15) & ~(size_t)15;
-              const size_t bytes = (hdr + (pay.size() + E.pay.size()) * 2 + 15) & ~(size_t)15;
-              if (bytes > (size_t)stage_bytes) {
-                if (na > 0) break;
-                return bail(8);   // one angle does not fit the staging buffer
-              }
-              const int shift = (int)pay.size();
-              for (int k = 0; k < 12; ++k) tbl.push_back(E.tbl[k] + shift);
-              pay.insert(pay.end(), E.pay.begin(), E.pay.end());
-              ++na;
+            segs.clear();
+            long used = 0;
+            while (a < ca0 + cna) {
+              const Encoded & E = enc[(size_t)a * nstage + sg];
+              const long room = ((long)stage_bytes - (long)((((segs.size() + 1) * 13) + 15) & ~(size_t)15)) / 64 - used;
+              if (room < 0 || (room == 0 && E.steps > k)) break;
+              const int take = (int)std::min<long>(E.steps - k, room);
+              segs.push_back({a, k, k + take});
+              used += take;
+              k += take;
+              if (k < E.steps) break;
+              ++a; k = 0;
             }
-            const size_t hdr = (((size_t)na * 52) + 15) & ~(size_t)15;
-            const size_t bytes = std::max<size_t>(16, (hdr + pay.size() * 2 + 15) & ~(size_t)15);
+            if (segs.empty()) return bail(8);   // the staging buffer holds no step
+            const int na = (int)segs.size();
+            const size_t hdr = (((size_t)na * 13) + 15) & ~(size_t)15;
+            const size_t bytes = hdr + (size_t)used * 64;
             TileSeq e{};
             e.off = (int32_t)blob.size();
             e.bytes = (int32_t)bytes;
-            e.chunk = (int16_t)v; e.stage = (int16_t)sg; e.a0 = (int16_t)a; e.na = (int16_t)na;
+            e.chunk = (int16_t)v; e.stage = (int16_t)sg; e.a0 = (int16_t)segs[0].a; e.na = (int16_t)na;
             e.flags = (first_sub ? kSeqNewStage : 0u) | ((first_sub && sg == 0) ? kSeqNewChunk : 0u);
-            for (int aa = a; aa < a + na; ++aa)
+            for (const Seg & sgm : segs)
               for (int m = 0; m < 4; ++m)
-                if (!egrp[((size_t)aa * nstage + sg) * 4 + m].empty()) e.flags |= kSeqHasEdge;
+                if (sgm.k0 == 0 && !egrp[((size_t)sgm.a * nstage + sg) * 4 + m].empty()) e.flags |= kSeqHasEdge;
             if (first_sub)
               for (int aa = ca0; aa < ca0 + cna; ++aa)
                 if (!wgrp[(size_t)aa * nstage + sg].empty()) e.flags |= kSeqHasWrap;
             blob.resize(blob.size() + bytes, 0);
-            if (na > 0) {
-              // (angle, alignment) groups by descending work: plain + multi descriptors + edge entries
-              std::vector<std::pair<int, int>> wt;
-              for (int g2 = 0; g2 < na * 4; ++g2) {
-                const int w = (tbl[3 * g2 + 1] - tbl[3 * g2]) + (tbl[3 * g2 + 2] - tbl[3 * g2 + 1]) / 2 +
-                              (int)egrp[((size_t)(a + (g2 >> 2)) * nstage + sg) * 4 + (g2 & 3)].size();
-                wt.emplace_back(-w, g2);
-              }
-              std::sort(wt.begin(), wt.end());
-              for (int g2 = 0; g2 < na * 4; ++g2) blob[e.off + (size_t)na * 48 + g2] = (uint8_t)wt[g2].second;
-              std::memcpy(blob.data() + e.off, tbl.data(), tbl.size() * 4);
-              if (!pay.empty()) std::memcpy(blob.data() + e.off + hdr, pay.data(), pay.size() * 2);
+            int32_t * tbl = reinterpret_cast<int32_t *>(blob.data() + e.off);
+            uint8_t * order = blob.data() + e.off + (size_t)na * 12;
+            uint32_t * steps = reinterpret_cast<uint32_t *>(blob.data() + e.off + hdr);
+            std::vector<std::pair<int, int>> wt;   // angles by descending stream length: the shared queue hands out long items first
+            int at = 0;
+            for (int i = 0; i < na; ++i) {
+              const Seg & sgm = segs[i];
+              const int len = sgm.k1 - sgm.k0;
+              tbl[3 * i + 0] = at; tbl[3 * i + 1] = at + len; tbl[3 * i + 2] = sgm.k0 == 0;
+              if (len) std::memcpy(steps + (size_t)at * 16, enc[(size_t)sgm.a * nstage + sg].pay.data() + (size_t)sgm.k0 * 16, (size_t)len * 64);
+              at += len;
+              wt.emplace_back(-len, i);
             }
+            std::sort(wt.begin(), wt.end());
+            for (int i = 0; i < na; ++i) order[i] = (uint8_t)wt[i].second;
             seq.push_back(e);
-            a += na;
             first_sub = false;
           } while (a < ca0 + cna);
         }

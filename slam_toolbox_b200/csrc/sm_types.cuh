@@ -159,7 +159,8 @@ struct TileDev {
   int enabled;
   int C, V, nAc;                 // cluster size, angle chunks, angles per chunk
   int nbands, band_rows, alloc_rows, pitch_w;   // sub-grid banding (rows of one parity), allocated rows, row pitch in words
-  int xtiles, ytiles;
+  int xtiles, ytiles;             // EDGE-beam items: x-tiles of 16 poses, y-tiles of 48 rows
+  int ygroups, wranges;          // FAST-beam items: 16-row slot groups, ranges of kTileSlots sub-grid words
   int stage_bytes;               // size of one descriptor staging buffer
   int nlevels;                   // distinct non-zero smear-kernel values if <= 4 (levelled raster without atomics), else 0
   uint32_t level[4];             // ... ascending
